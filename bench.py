@@ -11,7 +11,8 @@ A "step" is ONE allocate cycle (allocate.go:43-194) over the BASELINE config-3 s
            engine's stream, L2 flushed between steps.
   e2e    = same metric through the public C-ABI call sequence with HOST buffers:
            kb_session_load (host flatten + H2D) + kb_allocate (cycle + decisions D2H) per step, wall clock.
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  --dump-outputs DIR also writes the decisions of the last timed step as .npy files, so that
+two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -103,6 +104,18 @@ def parity_verdict(workload, eng, res, replica=0):
     if digest.state_digest(ns["idle"], ns["releasing"], osr["job_ready"], osr["job_share"]) != g["state"]:
         return "node/job state differs from the oracle digest"
     return "ok"
+
+
+DECISION_FIELDS = ("node", "kind", "dispatched", "step", "dispatch_step")
+
+
+def dump_outputs(out_dir, res):
+    """The decision table one kb_allocate hands its caller, one DIR/decisions_<field>.npy per field.  float64 holds every
+    int32 / uint32 value exactly; the largest workload (c5, 1M tasks) comes to 40 MB."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for f in DECISION_FIELDS:
+        np.save(os.path.join(out_dir, f"decisions_{f}.npy"), res.decisions[f].astype(np.float64))
 
 
 def cpu_sample(snap, conf, mode, threads, seconds, warm_tasks=0):
@@ -239,6 +252,8 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     t_wall1 = time.perf_counter()
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     if dist is not None:
         t = torch.tensor([dev_ms], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -405,7 +420,13 @@ def main():
                     help="N > 1: one cluster per GPU (weak scaling, default) or the same session on every GPU (strong)")
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="wall-time bound of each cpu_baseline sample")
     ap.add_argument("--ref-seconds", type=float, default=6.0, help="wall-time bound of one --impl reference step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the decisions of the last timed step (rank 0) as DIR/decisions_<field>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm runs bounded samples, not whole cycles")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     rank = int(os.environ.get("RANK", "0"))
